@@ -9,6 +9,7 @@ random-init weights of the named shapes (no network for checkpoints).  One "step
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA engine
     python bench.py --impl reference [...]                       # the reference algorithm (CPU oracle port) on host cores
+    python bench.py --dump-outputs DIR [...]                     # also write the last timed step's outputs to DIR/*.npy
 
 Prints ONE JSON line (rank 0).  `value` is measured with the prompt already resident in HBM; `e2e` goes through
 the public `EaModel.eagenerate` with a pinned-host prompt and host result (H2D/D2H inside the timed region).
@@ -28,6 +29,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -466,23 +468,33 @@ def tp_parity_check(world: int, rank: int, device: int):
 
 
 def timed_steps(m, prompt, steps, dist, gen_kw):
-    """K eagenerate calls bracketed by barrier + synchronize, timed with CUDA events on the engine's stream."""
+    """K eagenerate calls bracketed by barrier + synchronize, timed with CUDA events on the engine's stream.  Also returns what
+    the last call returned: (ids, new_token, idx)."""
     stream = m.cuda_stream()
     if dist is not None:
         dist.barrier()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
-    new_tokens, cycles = 0, 0
+    new_tokens, cycles, last = 0, 0, None
     for _ in range(steps):
-        _, nt, idx = m.eagenerate(prompt, max_new_tokens=NEW_TOKENS, max_length=2048, log=True, **gen_kw)
-        new_tokens += nt
-        cycles += idx + 1
+        last = m.eagenerate(prompt, max_new_tokens=NEW_TOKENS, max_length=2048, log=True, **gen_kw)
+        new_tokens += last[1]
+        cycles += last[2] + 1
     e1.record(stream)
     torch.cuda.synchronize()
     if dist is not None:
         dist.barrier()
-    return e0.elapsed_time(e1), new_tokens, cycles
+    return e0.elapsed_time(e1), new_tokens, cycles, last
+
+
+def dump_outputs(directory, ids, new_token, idx):
+    """Write what one `eagenerate(..., log=True)` call returns as float64 .npy files (token ids are exact in float64), so that
+    two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, value in (("ids", ids.cpu().numpy()), ("new_token", new_token), ("idx", idx)):
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(value, dtype=np.float64))
 
 
 def run_ours(args):
@@ -525,12 +537,14 @@ def run_ours(args):
     sampler = ClockSampler(local)
     sampler.start()
     log("timed region")
-    ms_dev, new_tokens, cycles = timed_steps(m, prompt_dev, args.steps, dist, gen_kw)   # inputs resident in HBM
+    ms_dev, new_tokens, cycles, last = timed_steps(m, prompt_dev, args.steps, dist, gen_kw)   # inputs resident in HBM
     st = m.stats()
     launches = st["kernel_launches"]
     chain_stats = {k: st[k] for k in ("chain_ms", "chain_bytes", "chain_launches")}
-    ms_e2e, new_tokens_e, _ = timed_steps(m, prompt_host, args.steps, dist, gen_kw)     # pinned-host prompt, host result
+    ms_e2e, new_tokens_e, _, _ = timed_steps(m, prompt_host, args.steps, dist, gen_kw)     # pinned-host prompt, host result
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     if dist is not None:
         t = torch.tensor([ms_dev, ms_e2e], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -680,7 +694,11 @@ def main():
     ap.add_argument("--cpu-cycles", type=int, default=6)
     ap.add_argument("--cpu-threads", type=int, default=0, help="threads of the CPU arm (0 = all effective cores)")
     ap.add_argument("--cpu-timeout", type=int, default=240)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last device-resident timed step returned (ids, new_token, idx) to DIR/<name>.npy as float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.dtype is None:
         args.dtype = MODELS[args.model]["dtype"]
     if args.impl == "reference":

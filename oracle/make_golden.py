@@ -150,6 +150,10 @@ def run_and_capture(m, em, prompt, sampling_seed=None, **gen_kw):
 
 from eagle_b200.synthetic import FIXTURES, base_fixture, fixture_models, make_prompt  # noqa: E402,F401  (the fixture registry lives with the weight factories)
 
+# Fixtures stored without the per-phase hidden states (head input `in_hidden`, verify features `hidden_new`): no test reads them
+# for these fixtures, and at the TP-8-shardable width they would take the file past 1 MB.
+NO_HIDDEN_STATES = {"e3_tp8_bf16"}
+
 
 # Stop conditions of the driver loop (ea_model.py:290-299).  The tokenizer's EOS / <|eot_id|> id is set to the token the greedy
 # golden run emits at the given index of its continuation, so the run must stop after the cycle that commits it.
@@ -301,6 +305,11 @@ def main():
         m, em = build_reference_model(tcfg, tW, hcfg, hW, eagle3, dtype, **tree)
         prompt = make_prompt(tcfg["vocab_size"], plen, pseed)
         rec = run_and_capture(m, em, prompt, sampling_seed=sseed, **gen_kw)
+        if fx in NO_HIDDEN_STATES:
+            for t in rec["trees"]:
+                del t["in_hidden"]
+            for c in rec["cycles"]:
+                c["hidden_new"] = None
         naive = m.naivegenerate(prompt, temperature=0.0, max_new_tokens=gen_kw["max_new_tokens"],
                                 max_length=gen_kw["max_length"]) if sseed is None else None
         rec["naive_ids"] = naive

@@ -43,6 +43,14 @@ def test_workload_names_identify_the_baseline_config():
     assert "configs[4]" in bench.baseline_config(_args("llama3-70b"))
 
 
+def test_dump_outputs_writes_the_call_result_as_float64(tmp_path):
+    import numpy as np
+    bench.dump_outputs(str(tmp_path / "out"), torch.tensor([[5, 128255, 7]]), 2, 1)
+    got = {n: np.load(tmp_path / "out" / f"{n}.npy") for n in ("ids", "new_token", "idx")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert got["ids"].tolist() == [[5.0, 128255.0, 7.0]] and float(got["new_token"]) == 2.0 and float(got["idx"]) == 1.0
+
+
 def test_closed_set_bigram_target_keeps_the_continuation_inside_the_draft_vocabulary():
     cfg = syn.target_config("tiny")
     W = syn.make_target_weights(cfg, 3, torch.bfloat16)
